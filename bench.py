@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- clouds/s of the PointNet++ (SSG) point-set-abstraction forward on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one inference forward of pointnet2_cls_ssg (FPS -> fused ball-query/group/MLP/max-pool x2 ->
 group-all MLP -> FC head, BN in moving-average mode) over one batch of B=32 synthetic clouds of N=2048 points
@@ -10,6 +10,8 @@ group-all MLP -> FC head, BN in moving-average mode) over one batch of B=32 synt
   e2e       same metric through the public API with HOST (pinned) buffers: H2D of the batch + forward + D2H logits;
   roofline  the dominant kernel of the step, timed live with CUDA events on the launching stream;
   cpu_baseline  the oracle port of the same forward on the host cores, on a bounded sample.
+`--dump-outputs DIR` writes the logits of the last timed step (rank 0) as DIR/logits.npy, float32 (B, 15).  Inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 `--impl reference` times only the CPU arm (there is no runnable TensorFlow here; see DESIGN.md).
 """
 from __future__ import annotations
@@ -334,6 +336,7 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the BGA / DGCNN / single-op / sweep measurements")
     ap.add_argument("--no-train", action="store_true", help="skip the training-step measurement")
     ap.add_argument("--train-steps", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's logits (rank 0) as DIR/logits.npy")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -385,9 +388,8 @@ def main():
     def timed(engine, host, steps, warmup):
         def step_fn(i):
             if host:
-                engine.submit(pool_host[i % POOL], to_host=True)    # pinned host batch in, logits back to pinned host memory
-            else:
-                engine.submit(pool_dev[i % POOL])                   # device-resident batch (rotating pool > L2)
+                return engine.submit(pool_host[i % POOL], to_host=True)    # pinned host batch in, logits back to pinned host memory
+            return engine.submit(pool_dev[i % POOL])                       # device-resident batch (rotating pool > L2)
         for i in range(warmup):
             step_fn(i)
         barrier()
@@ -396,24 +398,27 @@ def main():
         e0.record(main)
         engine.fence_begin(e0)
         for i in range(steps):
-            step_fn(warmup + i)
+            last = step_fn(warmup + i)
         engine.fence_end(main)
         e1.record(main)
         barrier()
-        return max_over_ranks(e0.elapsed_time(e1), device=dev)
+        return max_over_ranks(e0.elapsed_time(e1), device=dev), last       # ms, slot holding the last step's logits
 
     engine = pointnet2_cls_ssg_engine(params, batch=B, npoints=N, num_class=NUM_CLASS, slots=NSTREAMS, device=dev)
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_res = timed(engine, False, args.steps, args.warmup)
-    ms_e2e = timed(engine, True, args.steps, args.warmup)
+    ms_res, last_slot = timed(engine, False, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:           # read now: the host-buffer run below reuses the slots
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "logits.npy"), engine.result(last_slot).cpu().numpy().astype(np.float32))
+    ms_e2e, _ = timed(engine, True, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
     ms_res_1 = None
     if solo and NSTREAMS > 1:
         engine1 = pointnet2_cls_ssg_engine(params, batch=B, npoints=N, num_class=NUM_CLASS, slots=1, device=dev)
         n1 = max(args.steps // 4, 8)
-        ms_res_1 = timed(engine1, False, n1, args.warmup) / n1
+        ms_res_1 = timed(engine1, False, n1, args.warmup)[0] / n1
         del engine1
 
     train = run_training_bench(args, dev, rank, world, local_rank)

@@ -1,5 +1,6 @@
 """GPU parity: this repo's sm_100a kernels (through the C ABI via scanobjectnn_b200.ops) against
-(1) the CPU oracle and (2) the REFERENCE's own CUDA kernels compiled for sm_100a (oracle/_ref/libref_tfops.so).
+(1) the CPU oracle and (2) the REFERENCE's own CUDA kernels compiled for sm_100a, through the digests of their outputs on
+the same inputs (tests/golden/ref_gpu_ops.json, written by tests/golden/make_golden_ref.py on a B200).
 Index outputs must be bit-exact."""
 import numpy as np
 import pytest
@@ -9,10 +10,16 @@ from oracle import oracle as orc
 from scanobjectnn_b200 import ops
 from scanobjectnn_b200.synthetic import make_clouds
 
+from . import golden_util as golden
 from . import gpu_util as G
 
 pytestmark = pytest.mark.gpu
-needs_refgpu = pytest.mark.skipif(not orc.refgpu_available(), reason="oracle/_ref/libref_tfops.so not built")
+D = golden.digest
+
+
+def _ref(key):
+    """digests of the reference kernel's outputs for this test case"""
+    return golden.load("ref_gpu_ops.json")[key]
 
 
 # ----------------------------------------------------------------------------------------------- FPS
@@ -25,18 +32,14 @@ def test_fps_matches_oracle(kind, n, m):
     assert (got == orc.fps(xyz, m)).all()
 
 
-@needs_refgpu
 @pytest.mark.parametrize("kind,b,n,m", [("ball", 32, 2048, 512), ("dup", 32, 2048, 512), ("shell", 40, 512, 128),
                                         ("dup", 5, 4096, 256), ("ball", 2, 8192, 128), ("dup", 3, 700, 700)])
 def test_fps_matches_reference_kernel(kind, b, n, m):
     xyz = G.cu(make_clouds(kind, b, n, seed=7 + n))
     idx, new_xyz = ops.farthest_point_sample_and_gather(m, xyz)
-    ref = G.ref_fps(xyz, m)
-    assert torch.equal(idx, ref)
-    assert torch.equal(new_xyz, G.ref_gather_point(xyz, ref))
+    assert [D(idx), D(new_xyz)] == _ref(f"fps/{kind}/{b}/{n}/{m}")
 
 
-@needs_refgpu
 def test_fps_tie_break_and_oversampling():
     n = 1100
     xyz = np.zeros((2, n, 3), np.float32)
@@ -45,11 +48,11 @@ def test_fps_tie_break_and_oversampling():
     xyz[1, :, 1] = 0.25            # second cloud: same ties, shifted
     t = G.cu(xyz)
     got = ops.farthest_point_sample(5, t)
-    assert torch.equal(got, G.ref_fps(t, 5))
+    assert D(got) == _ref("fps_ties")
     assert G.npy(got)[0, :3].tolist() == [0, 512, 1024]
     # m > n: once every point is taken the reference keeps returning the (k mod 512, k)-minimal index
     small = G.cu(make_clouds("ball", 2, 5, seed=1))
-    assert torch.equal(ops.farthest_point_sample(9, small), G.ref_fps(small, 9))
+    assert D(ops.farthest_point_sample(9, small)) == _ref("fps_oversampled")
 
 
 def test_fps_nan_and_inf_inputs_match_oracle():
@@ -96,18 +99,15 @@ def test_ball_query_matches_oracle(kind, n, m, r, k):
     assert (G.npy(idx) == oi).all() and (G.npy(cnt) == oc).all()
 
 
-@needs_refgpu
 @pytest.mark.parametrize("kind,b,n,m,r,k", [("ball", 32, 2048, 512, 0.2, 32), ("shell", 32, 2048, 512, 0.2, 64),
                                             ("dup", 32, 512, 128, 0.4, 64), ("ball", 4, 4096, 1024, 0.1, 16)])
 def test_ball_query_matches_reference_kernel(kind, b, n, m, r, k):
     xyz = G.cu(make_clouds(kind, b, n, seed=n + k + 1))
     q = ops.gather_point(xyz, ops.farthest_point_sample(m, xyz))
     idx, cnt = ops.query_ball_point(r, k, xyz, q)
-    ridx, rcnt = G.ref_query_ball_point(r, k, xyz, q)
-    assert torch.equal(idx, ridx) and torch.equal(cnt, rcnt)
+    assert [D(idx), D(cnt)] == _ref(f"ball_query/{kind}/{b}/{n}/{m}/{r}/{k}")
 
 
-@needs_refgpu
 def test_ball_query_radius_boundary_and_specials():
     # distances that land exactly on / next to the radius: lattice points at multiples of 0.05 from the query
     g = np.arange(-8, 9, dtype=np.float32) * np.float32(0.05)
@@ -118,9 +118,7 @@ def test_ball_query_radius_boundary_and_specials():
     xt, qt = G.cu(xyz), G.cu(q)
     for r in (0.05, 0.1, 0.15, 0.2, 0.25, 0.3, 0.0707, 0.0866, np.nextafter(np.float32(0.2), np.float32(1))):
         idx, cnt = ops.query_ball_point(float(r), 64, xt, qt)
-        ridx, rcnt = G.ref_query_ball_point(float(r), 64, xt, qt)
-        assert torch.equal(cnt, rcnt), r
-        assert torch.equal(idx, ridx), r
+        assert [D(idx), D(cnt)] == _ref(f"ball_query_radius/{float(r)!r}"), r
     # NaN / inf coordinates in the dataset: CUDA's max(NaN,1e-20f) makes a NaN distance count as inside
     x2 = make_clouds("ball", 2, 200, seed=3)
     x2[0, 5] = np.nan
@@ -128,8 +126,7 @@ def test_ball_query_radius_boundary_and_specials():
     xt2 = G.cu(x2)
     qt2 = G.cu(x2[:, 20:40].copy())
     idx, cnt = ops.query_ball_point(0.3, 16, xt2, qt2)
-    ridx, rcnt = G.ref_query_ball_point(0.3, 16, xt2, qt2)
-    assert torch.equal(idx, ridx) and torch.equal(cnt, rcnt)
+    assert [D(idx), D(cnt)] == _ref("ball_query_nonfinite")
 
 
 def test_ball_query_empty_ball_and_errors():
@@ -154,8 +151,7 @@ def test_group_point_and_grad(c):
     t = G.cu(pts).requires_grad_(True)
     out = ops.group_point(t, G.cu(idx))
     assert np.array_equal(G.npy(out), orc.group_point(pts, idx))
-    if orc.refgpu_available():
-        assert torch.equal(out.detach(), G.ref_group_point(t.detach(), G.cu(idx)))
+    assert D(out) == _ref(f"group_point/{c}")
     go = rng.standard_normal(out.shape).astype(np.float32)
     out.backward(G.cu(go))
     assert np.array_equal(G.npy(t.grad), orc.group_point_grad(pts.shape, idx, go))
@@ -175,9 +171,7 @@ def test_selection_sort_kat_and_oracle():
         oi, ov = orc.selection_sort(k, d)
         gi, gv = ops.select_top_k(k, G.cu(d))
         assert np.array_equal(G.npy(gi), oi) and np.array_equal(G.npy(gv), ov, equal_nan=True)
-        if orc.refgpu_available():
-            ri, rv = G.ref_selection_sort(k, G.cu(d))
-            assert torch.equal(gi, ri) and np.array_equal(G.npy(gv), G.npy(rv), equal_nan=True)
+        assert [D(gi), D(gv)] == _ref(f"selection_sort/{k}"), k
 
 
 @pytest.mark.parametrize("kind", ["ball", "dup"])

@@ -1,13 +1,19 @@
-"""Pin the CPU restatement (oracle/psa_oracle.c) against the reference's OWN code compiled here
-(oracle/_ref/libref_cpu.so, built by `make -C oracle ref` from /root/reference) and against the
-reference's only deterministic known-answer test (grouping/test/selection_sort.cpp:68-78)."""
+"""Pin the CPU restatement (oracle/psa_oracle.c) against the reference's OWN CPU code (the digests of its outputs on these
+inputs, tests/golden/ref_cpu_pins.json, written by tests/golden/make_golden_ref.py) and against the reference's only
+deterministic known-answer test (grouping/test/selection_sort.cpp:68-78)."""
 import numpy as np
 import pytest
 
 from oracle import oracle as orc
 from scanobjectnn_b200.synthetic import make_clouds
 
-needs_ref = pytest.mark.skipif(not orc.refcpu_available(), reason="oracle/_ref/libref_cpu.so not built")
+from . import golden_util as golden
+
+D = golden.digest
+
+
+def _ref(key):
+    return golden.load("ref_cpu_pins.json")[key]
 
 
 def test_selection_sort_kat():
@@ -21,7 +27,6 @@ def test_selection_sort_kat():
     assert (outi == np.array([3, 2, 1, 0])).all()
 
 
-@needs_ref
 def test_selection_sort_matches_reference_cpu():
     rng = np.random.default_rng(5)
     dist = rng.random((3, 7, 50), dtype=np.float32)
@@ -29,64 +34,52 @@ def test_selection_sort_matches_reference_cpu():
     dist[1, 2, :] = 0.5
     for k in (1, 5, 50):
         oi, ov = orc.selection_sort(k, dist)
-        ri, rv = orc.refcpu_selection_sort(k, dist)
-        assert (oi == ri).all() and (ov == rv).all()
+        assert [D(oi), D(ov)] == _ref(f"selection_sort/{k}"), k
 
 
-@needs_ref
 @pytest.mark.parametrize("kind", ["ball", "shell", "dup"])
 def test_ball_query_matches_reference_cpu(kind):
     xyz = make_clouds(kind, 4, 512, seed=11)
     q = xyz[:, ::4, :].copy()
     for r, k in ((0.1, 64), (0.2, 32), (0.4, 16)):
         oi, cnt = orc.query_ball_point(r, k, xyz, q, contract=False, fill=-7)
-        ri = orc.refcpu_query_ball_point(r, k, xyz, q, fill=-7)
-        assert (oi == ri).all()
+        assert D(oi) == _ref(f"ball_query/{kind}/{r}/{k}"), (r, k)
         assert cnt.min() >= 1          # queries are dataset points: self-distance 1e-20 < r
 
 
-@needs_ref
 def test_ball_query_empty_ball_leaves_row_untouched():
     xyz = make_clouds("ball", 2, 64, seed=3)
     q = np.full((2, 5, 3), 9.0, np.float32)
     oi, cnt = orc.query_ball_point(0.2, 8, xyz, q, contract=False, fill=-7)
-    ri = orc.refcpu_query_ball_point(0.2, 8, xyz, q, fill=-7)
-    assert (oi == -7).all() and (ri == -7).all() and (cnt == 0).all()
+    assert (oi == -7).all() and (cnt == 0).all()
+    assert D(oi) == _ref("ball_query_empty")                # the reference leaves the row untouched too
 
 
-@needs_ref
 def test_group_point_and_grad_match_reference_cpu():
     rng = np.random.default_rng(9)
     pts = rng.standard_normal((3, 40, 7)).astype(np.float32)
     idx = rng.integers(0, 40, size=(3, 11, 5), dtype=np.int32)
-    assert (orc.group_point(pts, idx) == orc.refcpu_group_point(pts, idx)).all()
     go = rng.standard_normal((3, 11, 5, 7)).astype(np.float32)
-    assert (orc.group_point_grad(pts.shape, idx, go) == orc.refcpu_group_point_grad(pts.shape, idx, go)).all()
+    assert [D(orc.group_point(pts, idx)), D(orc.group_point_grad(pts.shape, idx, go))] == _ref("group_point")
 
 
-@needs_ref
 @pytest.mark.parametrize("n,m", [(128, 1), (128, 2), (512, 128), (300, 77)])
 def test_three_nn_matches_reference_cpu(n, m):
     xyz1 = make_clouds("shell", 3, n, seed=21)
     xyz2 = make_clouds("dup", 3, max(m, 4), seed=22)[:, :m, :].copy()
     od, oi = orc.three_nn(xyz1, xyz2)
-    rd, ri = orc.refcpu_three_nn(xyz1, xyz2)
-    assert (oi == ri).all()
-    assert np.array_equal(od, rd)          # inf == inf for the m<3 slots
+    assert [D(od), D(oi)] == _ref(f"three_nn/{n}/{m}")     # inf == inf for the m<3 slots
     if m < 3:
         assert np.isinf(od[..., m:]).all() and (oi[..., m:] == 0).all()
 
 
-@needs_ref
 def test_three_interpolate_and_grad_match_reference_cpu():
     rng = np.random.default_rng(2)
     pts = rng.standard_normal((2, 30, 9)).astype(np.float32)
     idx = rng.integers(0, 30, size=(2, 50, 3), dtype=np.int32)
     w = rng.random((2, 50, 3), dtype=np.float32)
-    assert np.array_equal(orc.three_interpolate(pts, idx, w), orc.refcpu_three_interpolate(pts, idx, w))
     go = rng.standard_normal((2, 50, 9)).astype(np.float32)
-    assert np.array_equal(orc.three_interpolate_grad(pts.shape, idx, w, go),
-                          orc.refcpu_three_interpolate_grad(pts.shape, idx, w, go))
+    assert [D(orc.three_interpolate(pts, idx, w)), D(orc.three_interpolate_grad(pts.shape, idx, w, go))] == _ref("three_interpolate")
 
 
 def test_fps_basic_properties():

@@ -1,25 +1,23 @@
-"""GPU-vs-GPU: the reference's own CUDA kernels (compiled unmodified for sm_100a, oracle/_ref/libref_tfops.so) timed beside
-the libpsa kernels on identical tensors at the SSG shapes (SURVEY 8d "timing the ref beside it").  Same outputs (index-exact,
-checked here again), CUDA-event medians.  The table goes to gpurun_out/ref_gpu_compare.json; profiles/ keeps a copy."""
-import ctypes as C
+"""GPU-vs-GPU: the libpsa kernels against the reference's own CUDA kernels (compiled unmodified for sm_100a) at the SSG shapes
+(SURVEY 8d "timing the ref beside it").  tests/golden/make_golden_ref.py ran the reference's kernels on the same seeded inputs on a
+B200 and stored their output digests and CUDA-event medians in tests/golden/ref_gpu_ops.json, with the GPU's name and power limit.
+Here the outputs must be identical (index-exact) and every kernel faster than the reference's stored time."""
 import json
-import os
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import oracle as orc
 from scanobjectnn_b200 import ops
 from scanobjectnn_b200.synthetic import make_clouds
+from tests import golden_util as golden
 from tests import gpu_util as G
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not orc.refgpu_available(), reason="oracle/_ref/libref_tfops.so not built")]
+pytestmark = pytest.mark.gpu
+B = 32
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-
-def _time(fn, reps=7, warm=2):
+def time_us(fn, reps=7, warm=2):
     for _ in range(warm):
         fn()
     ts = []
@@ -33,78 +31,51 @@ def _time(fn, reps=7, warm=2):
     return ts[len(ts) // 2]
 
 
+def ssg_inputs():
+    """seeded: B=32 clouds of 2048 points, SA2 features (B,512,128), a (B,128,512) distance matrix for SelectionSort"""
+    rng = np.random.default_rng(1001)
+    return (G.cu(make_clouds("ball", B, 2048, seed=1001)), G.cu(rng.standard_normal((B, 512, 128), dtype=np.float32)),
+            G.cu(rng.random((B, 128, 512), dtype=np.float32)))
+
+
 def test_libpsa_kernels_beat_the_reference_kernels():
-    B = 32
-    ref = orc.refgpu()
-    p = lambda t: C.c_void_p(t.data_ptr())
-    xyz = G.cu(make_clouds("ball", B, 2048, seed=1001))
+    gold = golden.load("ref_gpu_ops.json")
+    xyz, feats, dist = ssg_inputs()
+    out = {}
     rows = {}
 
-    def case(name, ours, theirs, check):
-        t_ours, t_ref = _time(ours), _time(theirs)
-        check()
-        rows[name] = {"libpsa_us": round(t_ours, 1), "reference_kernel_us": round(t_ref, 1), "speedup": round(t_ref / t_ours, 2)}
+    def case(name, ours, outs):
+        t_ours, t_ref = time_us(ours), gold["reference_kernel_us"][name]
+        assert [golden.digest(o) for o in outs()] == gold[f"ssg/{name}"], f"{name}: output differs from the reference kernel's"
+        rows[name] = {"libpsa_us": round(t_ours, 1), "reference_kernel_us": t_ref, "speedup": round(t_ref / t_ours, 2)}
 
-    # FPS (+ gather) at SA1 and SA2
-    temp = torch.empty((32, 2048), dtype=torch.float32, device="cuda")
-    ridx1 = torch.zeros((B, 512), dtype=torch.int32, device="cuda")
-    rnew1 = torch.zeros((B, 512, 3), dtype=torch.float32, device="cuda")
-    def ref_fps1():
-        ref.ref_fps(B, 2048, 512, p(xyz), p(temp), p(ridx1), 0)
-        ref.ref_gather_point(B, 2048, 512, p(xyz), p(ridx1), p(rnew1), 0)
-    out = {}
-    def our_fps1():
+    def fps1():
         out["i1"], out["x1"] = ops.farthest_point_sample_and_gather(512, xyz)
-    case("fps+gather 2048->512", our_fps1, ref_fps1, lambda: (torch.equal(out["i1"], ridx1) and torch.equal(out["x1"], rnew1)) or pytest.fail("fps1 mismatch"))
+    case("fps+gather 2048->512", fps1, lambda: [out["i1"], out["x1"]])
     l1 = out["x1"].contiguous()
-    ridx2 = torch.zeros((B, 128), dtype=torch.int32, device="cuda")
-    rnew2 = torch.zeros((B, 128, 3), dtype=torch.float32, device="cuda")
-    def ref_fps2():
-        ref.ref_fps(B, 512, 128, p(l1), p(temp), p(ridx2), 0)
-        ref.ref_gather_point(B, 512, 128, p(l1), p(ridx2), p(rnew2), 0)
-    def our_fps2():
+
+    def fps2():
         out["i2"], out["x2"] = ops.farthest_point_sample_and_gather(128, l1)
-    case("fps+gather 512->128", our_fps2, ref_fps2, lambda: torch.equal(out["i2"], ridx2) or pytest.fail("fps2 mismatch"))
+    case("fps+gather 512->128", fps2, lambda: [out["i2"], out["x2"]])
     l2 = out["x2"].contiguous()
 
-    # ball query at SA1 / SA2
-    for name, (r, k, a, q) in {"query_ball_point r=0.2 k=32 (2048, 512)": (0.2, 32, xyz, l1), "query_ball_point r=0.4 k=64 (512, 128)": (0.4, 64, l1, l2)}.items():
-        n, m = a.shape[1], q.shape[1]
-        ri = torch.zeros((B, m, k), dtype=torch.int32, device="cuda")
-        rc = torch.zeros((B, m), dtype=torch.int32, device="cuda")
-        def theirs(r=r, k=k, a=a, q=q, n=n, m=m, ri=ri, rc=rc):
-            ref.ref_query_ball_point(B, n, m, C.c_float(r), k, p(a), p(q), p(ri), p(rc), 0)
+    for name, (r, k, a, q) in {"query_ball_point r=0.2 k=32 (2048, 512)": (0.2, 32, xyz, l1),
+                               "query_ball_point r=0.4 k=64 (512, 128)": (0.4, 64, l1, l2)}.items():
         def ours(r=r, k=k, a=a, q=q, key=name):
             out[key] = ops.query_ball_point(r, k, a, q)
-        case(name, ours, theirs, lambda key=name, ri=ri, rc=rc: (torch.equal(out[key][0], ri) and torch.equal(out[key][1], rc)) or pytest.fail(key))
+        case(name, ours, lambda key=name: list(out[key]))
     idx2 = out["query_ball_point r=0.4 k=64 (512, 128)"][0]
 
     # group_point at the SA2 size (the tensor the fused path never writes): (B,512,128) by (B,128,64)
-    feats = torch.randn((B, 512, 128), device="cuda")
-    rg = torch.empty((B, 128, 64, 128), dtype=torch.float32, device="cuda")
-    def ref_group():
-        ref.ref_group_point(B, 512, 128, 128, 64, p(feats), p(idx2), p(rg), 0)
-    def our_group():
+    def group():
         out["g"] = ops.group_point(feats, idx2)
-    case("group_point C=128 (128 MiB out)", our_group, ref_group, lambda: torch.equal(out["g"], rg) or pytest.fail("group mismatch"))
+    case("group_point C=128 (128 MiB out)", group, lambda: [out["g"]])
 
-    # the whole SA2 level: reference = group xyz + group feats (its cuDNN convs are not available) vs the fused level
-    # -> reported as context only: ref_group above is a LOWER bound on the reference's level time.
     # SelectionSort (knn_point's op) at b*m = 4096 rows of 512
-    dist = torch.rand((B, 128, 512), device="cuda")
-    ro, rv = torch.empty((B, 128, 512), dtype=torch.int32, device="cuda"), torch.empty((B, 128, 512), dtype=torch.float32, device="cuda")
-    def ref_sel():
-        ref.ref_selection_sort(B, 512, 128, 32, p(dist), p(ro), p(rv), 0)
-    def our_sel():
+    def sel():
         out["s"] = ops.select_top_k(32, dist)
-    case("selection_sort k=32 (4096 rows x 512)", our_sel, ref_sel, lambda: torch.equal(out["s"][0][..., :32], ro[..., :32]) or pytest.fail("selection mismatch"))
+    case("selection_sort k=32 (4096 rows x 512)", sel, lambda: [out["s"][0][..., :32]])
 
-    print(json.dumps(rows, indent=1))
-    try:
-        os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-        with open(os.path.join(ROOT, "gpurun_out", "ref_gpu_compare.json"), "w") as f:
-            json.dump(rows, f, indent=1)
-    except OSError:
-        pass
+    print(json.dumps({"reference_measured_on": gold["measured_on"], **rows}, indent=1))
     slow = {k: v for k, v in rows.items() if v["speedup"] < 1.0}
     assert not slow, f"slower than the reference kernel: {slow}"
