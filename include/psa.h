@@ -395,6 +395,43 @@ PSA_API int psa_sa_conv1_bwd(int b, int n, int m, int nsample, int C1, const flo
                              const int* idx, const psa_grad_in* g, float* dW_xyz, float* dU, void* workspace,
                              size_t workspace_bytes, psa_stream_t stream);
 
+/* Training-mode front of a feature-propagation module (pointnet2/utils/pointnet_util.py:199-229 with three_nn / three_interpolate,
+ * 3d_interpolation/tf_interpolate.cpp:60-127, inside pointnet2/models/pointnet2_cls_bga.py:51-53).  The first 1x1 conv of the module
+ * distributes over the (linear) interpolation:
+ *   y = [interp, skip] . W1 + b = sum_i w_i U[idx_i] + skip . W1[C_a:] + b,   U = P2 . W1[:C_a]  (one row per KNOWN point)
+ * so the (b, n, C_a) interpolated tensor and the concatenation never exist.  U (b, m, C1) comes from psa_train_dense_fwd (its
+ * psa_act_in applies the producer's batch norm + relu on load), as does the skip product.  This call does, in one pass:
+ * three_nn of xyz1 (b,n,3) unknown against xyz2 (b,m,3) known + the inverse-distance weights (arithmetic and results bit-identical to
+ * psa_three_nn_interpolate), pre (b,n,C1) = [pre if accumulate, else bias (or 0 for NULL)] + (U[i1] w1 + U[i2] w2) + U[i3] w3,
+ * idx / weight (b,n,3) for the backward, and, if stats != NULL, stats (2, C1) = per-channel [sum, sum of squares] of pre (fixed-order
+ * CTA partials added in fp64).  Slots beyond m (m < 3) have weight 0 and idx 0.  C1 a multiple of 4, at most 512; m >= 1.
+ * workspace: psa_fp_conv1_prebn_workspace_bytes(b, n, C1) when stats != NULL. */
+PSA_API size_t psa_fp_conv1_prebn_workspace_bytes(int b, int n, int C1);
+PSA_API int psa_fp_conv1_prebn(int b, int n, int m, int C1, const float* xyz1, const float* xyz2, const float* U, const float* bias,
+                               int accumulate, float* pre, int* idx, float* weight, float* stats, void* workspace,
+                               size_t workspace_bytes, psa_stream_t stream);
+
+/* Backward of psa_fp_conv1_prebn: dU (b, m, C1) = ThreeInterpolateGrad(dy0, idx, weight) (tf_interpolate.cpp:131-153), dy0 = g over the
+ * b*n unknown rows (mode 0, evaluated on load: the batch-norm backward coefficients are applied there).  Ordered like
+ * psa_three_interpolate_grad (stable counting sort by destination, each known point adds round(dy0 * w) of its entries 3*row + slot
+ * in ascending order): with a plain g (dy0 = dh) the result is bit-identical to psa_three_interpolate_grad(dh).  The rest of the
+ * layer's backward is dense: dW1[:C_a] = P2^T . dU and dP2 = dU . W1[:C_a]^T over the b*m known points, dW1[C_a:] = skip^T . dy0 and
+ * dskip = psa_train_dense_bwd_input(..., col_skip = C_a).  workspace: psa_fp_conv1_bwd_workspace_bytes(b, n, m). */
+PSA_API size_t psa_fp_conv1_bwd_workspace_bytes(int b, int n, int m);
+PSA_API int psa_fp_conv1_bwd(int b, int n, int m, int C1, const int* idx, const float* weight, const psa_grad_in* g, float* dU,
+                             void* workspace, size_t workspace_bytes, psa_stream_t stream);
+
+/* Joint loss of pointnet2_cls_bga.get_loss (pointnet2/models/pointnet2_cls_bga.py:78-93): class logits (b, c) with labels (b) int32,
+ * per-point seg logits (b, n, 2) with a binary mask (b, n) int32 ->
+ *   loss (3) = [(1-w) classify + w seg, classify = mean_b CE, seg = mean over b*n points of the 2-way CE],
+ *   dcls (b, c) = (1-w) (softmax - onehot) / b,  dseg (b, n, 2) = w (softmax - onehot) / (b n).
+ * Sums in a fixed order (per-block trees, blocks added in order, fp64).  A label or mask value outside its range gives NaN.
+ * workspace: psa_cls_seg_xent_workspace_bytes(b, n). */
+PSA_API size_t psa_cls_seg_xent_workspace_bytes(int b, int n);
+PSA_API int psa_cls_seg_xent(int b, int c, int n, const float* cls_logits, const int* labels, const float* seg_logits, const int* mask,
+                             float seg_weight, float* loss, float* dcls, float* dseg, void* workspace, size_t workspace_bytes,
+                             psa_stream_t stream);
+
 /* Mean sparse softmax cross-entropy (pointnet2_cls_ssg.py:50-57) and its gradient: logits (b, c), labels (b) int32 ->
  * loss (1), dlogits (b, c) = (softmax - onehot) / b. */
 PSA_API int psa_softmax_xent(int b, int c, const float* logits, const int* labels, float* loss, float* dlogits,

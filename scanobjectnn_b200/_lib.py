@@ -88,6 +88,9 @@ SIGNATURES = {
     "psa_train_pool_fwd": [_ll, _i, _i, _p, _p, _p, _p, _p, _p],
     "psa_bn_bwd_coeffs": [_ll, _i, _gin, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p],
     "psa_sa_conv1_bwd": [_i, _i, _i, _i, _i, _p, _p, _p, _gin, _p, _p, _p, _sz, _p],
+    "psa_fp_conv1_prebn": [_i, _i, _i, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _sz, _p],
+    "psa_fp_conv1_bwd": [_i, _i, _i, _i, _p, _p, _gin, _p, _p, _sz, _p],
+    "psa_cls_seg_xent": [_i, _i, _i, _p, _p, _p, _p, _f, _p, _p, _p, _p, _sz, _p],
     "psa_softmax_xent": [_i, _i, _p, _p, _p, _p, _p],
     "psa_pool_rows": [_ll, _i, _i, _i, _p, _p, _p, _p],
     "psa_adam_step": [_ll, _p, _p, _p, _p, _f, _f, _f, _f, _i, _f, _p],
@@ -95,7 +98,8 @@ SIGNATURES = {
 INFO_SYMBOLS = ("psa_version", "psa_last_error", "psa_sm_arch", "psa_shared_mlp_workspace_bytes",
                 "psa_sa_module_workspace_bytes", "psa_sa_conv1_prebn_workspace_bytes", "psa_sa_group_all_workspace_bytes", "psa_edgeconv_workspace_bytes",
                 "psa_train_dense_workspace_bytes", "psa_bn_bwd_workspace_bytes", "psa_sa_conv1_bwd_workspace_bytes", "psa_knn_graph_workspace_bytes",
-                "psa_scatter_workspace_bytes")
+                "psa_scatter_workspace_bytes", "psa_fp_conv1_prebn_workspace_bytes", "psa_fp_conv1_bwd_workspace_bytes",
+                "psa_cls_seg_xent_workspace_bytes")
 
 _lib = None
 
@@ -134,6 +138,10 @@ def load() -> C.CDLL:
     lib.psa_knn_graph_workspace_bytes.restype = C.c_size_t
     lib.psa_scatter_workspace_bytes.argtypes = [_i, _i, _ll]
     lib.psa_scatter_workspace_bytes.restype = C.c_size_t
+    for name, argtypes in (("psa_fp_conv1_prebn_workspace_bytes", [_i, _i, _i]), ("psa_fp_conv1_bwd_workspace_bytes", [_i, _i, _i]),
+                           ("psa_cls_seg_xent_workspace_bytes", [_i, _i])):
+        getattr(lib, name).argtypes = argtypes
+        getattr(lib, name).restype = C.c_size_t
     lib.psa_version.restype = C.c_int
     lib.psa_sm_arch.restype = C.c_int
     lib.psa_last_error.restype = C.c_char_p

@@ -406,10 +406,43 @@ class PointNet2ClsTrainer(_TrainOps):
                 ly.mask.copy_((r < keep).to(torch.float32) / keep)
 
     # ------------------------------------------------------------------------------------------------
+    def _level_forward(self, lv: _Level, cur_xyz: torch.Tensor, cur_pts: torch.Tensor | None, bn_decay: float):
+        """one set-abstraction level in training mode: lv.new_xyz, the layers' pre-BN activations, lv.pooled"""
+        lib = self.lib
+        B = self.B
+        sp = lv.spec
+        L0 = lv.layers[0]
+        if sp.group_all:
+            # sample_and_group_all (pointnet_util.py:59-84): rows = [xyz, points], one group per cloud
+            lv.x_cat[:, :3].copy_(cur_xyz.reshape(-1, 3))
+            if cur_pts is not None:
+                lv.x_cat[:, 3:].copy_(cur_pts.reshape(B * lv.n, -1))
+            self._dense_fwd(L0, _raw_in(lv.x_cat))
+            lv.new_xyz = torch.zeros((B, 1, 3), dtype=torch.float32, device=self.dev)
+        else:
+            _, lv.new_xyz = ops.farthest_point_sample_and_gather(lv.m, cur_xyz)
+            self._c(lib.psa_sa_conv1_prebn(B, lv.n, lv.m, lv.c_in, C.c_float(sp.radius), lv.k, _p(cur_xyz), _p(lv.new_xyz), _p(cur_pts),
+                                           _p(L0.W), _p(L0.b), L0.N, _p(L0.y), _p(lv.idx), _p(lv.cnt), _p(L0.stats), _p(self.ws),
+                                           C.c_size_t(self.ws_bytes), _stream()), "sa_conv1_prebn")
+        self._bn_finalize(L0, L0.rows, bn_decay)
+        prev = L0
+        for ly in lv.layers[1:]:
+            self._dense_fwd(ly, prev.act_in())
+            self._bn_finalize(ly, ly.rows, bn_decay)
+            prev = ly
+        self._c(lib.psa_train_pool_fwd(B * lv.m, lv.k, prev.N, _p(prev.y), _p(prev.scale), _p(prev.shift), _p(lv.pooled), _p(lv.argk),
+                                       _stream()), "train_pool_fwd")
+
     def forward(self, xyz: torch.Tensor, bn_decay: float = 0.5, points: torch.Tensor | None = None) -> torch.Tensor:
         """Training-mode forward (batch statistics, moving averages updated with `bn_decay`) -> logits (B, num_class); without a head
         -> the last level's pooled features (B*m, C).  `points` (B, N, in_channels): input features of the first level."""
-        lib = self.lib
+        feat = self._levels_forward(xyz, points, bn_decay)
+        if not self.head:
+            return feat
+        return self._head_forward(feat, bn_decay)
+
+    def _levels_forward(self, xyz: torch.Tensor, points: torch.Tensor | None, bn_decay: float) -> torch.Tensor:
+        """the set-abstraction levels -> the last level's pooled features"""
         B = self.B
         assert xyz.shape == (B, self.N0, 3) and xyz.is_cuda and xyz.dtype == torch.float32
         assert (points is None) == (self.in_channels == 0), "points must be given exactly when the trainer was built with in_channels > 0"
@@ -419,33 +452,13 @@ class PointNet2ClsTrainer(_TrainOps):
             cur_pts = points.contiguous()
         self.in_xyz = []
         for lv in self.levels:
-            sp = lv.spec
             self.in_xyz.append((cur_xyz, cur_pts))
-            L0 = lv.layers[0]
-            if sp.group_all:
-                # sample_and_group_all (pointnet_util.py:59-84): rows = [xyz, points], one group per cloud
-                lv.x_cat[:, :3].copy_(cur_xyz.reshape(-1, 3))
-                if cur_pts is not None:
-                    lv.x_cat[:, 3:].copy_(cur_pts.reshape(B * lv.n, -1))
-                self._dense_fwd(L0, _raw_in(lv.x_cat))
-                lv.new_xyz = torch.zeros((B, 1, 3), dtype=torch.float32, device=self.dev)
-            else:
-                _, lv.new_xyz = ops.farthest_point_sample_and_gather(lv.m, cur_xyz)
-                self._c(lib.psa_sa_conv1_prebn(B, lv.n, lv.m, lv.c_in, C.c_float(sp.radius), lv.k, _p(cur_xyz), _p(lv.new_xyz), _p(cur_pts),
-                                               _p(L0.W), _p(L0.b), L0.N, _p(L0.y), _p(lv.idx), _p(lv.cnt), _p(L0.stats), _p(self.ws),
-                                               C.c_size_t(self.ws_bytes), _stream()), "sa_conv1_prebn")
-            self._bn_finalize(L0, L0.rows, bn_decay)
-            prev = L0
-            for ly in lv.layers[1:]:
-                self._dense_fwd(ly, prev.act_in())
-                self._bn_finalize(ly, ly.rows, bn_decay)
-                prev = ly
-            self._c(lib.psa_train_pool_fwd(B * lv.m, lv.k, prev.N, _p(prev.y), _p(prev.scale), _p(prev.shift), _p(lv.pooled), _p(lv.argk),
-                                           _stream()), "train_pool_fwd")
+            self._level_forward(lv, cur_xyz, cur_pts, bn_decay)
             cur_xyz, cur_pts = lv.new_xyz, lv.pooled.view(B, lv.m, -1)
-        feat = self.levels[-1].pooled                                   # (B, C)
-        if not self.head:
-            return feat
+        return self.levels[-1].pooled
+
+    def _head_forward(self, feat: torch.Tensor, bn_decay: float) -> torch.Tensor:
+        """the FC head on the global feature (B, C) -> logits"""
         a = _raw_in(feat)
         for ly in self.head:
             self._dense_fwd(ly, a)
@@ -455,10 +468,49 @@ class PointNet2ClsTrainer(_TrainOps):
         return self.head[-1].y
 
     # ------------------------------------------------------------------------------------------------
-    def backward(self, dlogits: torch.Tensor):
-        """Gradients of every trainable variable for d(loss)/d(logits) = dlogits, into the flat gradient bucket."""
+    def _level_backward(self, li: int, dpool: torch.Tensor):
+        """gradients of level li's variables for d(loss)/d(pooled) = dpool; the gradient of its input features goes to lv.d_in"""
         lib = self.lib
         B = self.B
+        lv = self.levels[li]
+        sp = lv.spec
+        L = len(lv.layers)
+        cur_xyz, cur_pts = self.in_xyz[li]
+        for l in range(L - 1, 0, -1):
+            ly = lv.layers[l]
+            if l == L - 1:
+                g0 = _grad_pooled(ly, dpool, lv.pooled, lv.argk, lv.k, False)
+                g1 = _grad_pooled(ly, dpool, lv.pooled, lv.argk, lv.k, True)
+            else:
+                g0 = _grad_dense(ly, lv.dh[l], False)
+                g1 = _grad_dense(ly, lv.dh[l], True)
+            self._layer_bwd(ly, g0, g1, lv.layers[l - 1].act_in(), lv.dh[l - 1])
+        L0 = lv.layers[0]
+        if L == 1:
+            g0 = _grad_pooled(L0, dpool, lv.pooled, lv.argk, lv.k, False)
+            g1 = _grad_pooled(L0, dpool, lv.pooled, lv.argk, lv.k, True)
+        else:
+            g0 = _grad_dense(L0, lv.dh[0], False)
+            g1 = _grad_dense(L0, lv.dh[0], True)
+        if sp.group_all:
+            self._layer_bwd(L0, g0, g1, _raw_in(lv.x_cat), lv.d_in, col_skip=3)
+        else:
+            self._c(lib.psa_bn_bwd_coeffs(L0.rows, L0.N, C.byref(g0), _p(L0.gamma), _p(L0.mean_inv), _p(L0.dgamma), _p(L0.dbeta),
+                                          _p(L0.ca), _p(L0.cb), _p(L0.cc), _p(self.ws), C.c_size_t(self.ws_bytes), _stream()), "bn_bwd_coeffs")
+            L0.db.zero_()
+            self._c(lib.psa_sa_conv1_bwd(B, lv.n, lv.m, lv.k, L0.N, _p(cur_xyz), _p(lv.new_xyz), _p(lv.idx), C.byref(g1), _p(L0.dW[:3]),
+                                         _p(lv.dU), _p(self.ws), C.c_size_t(self.ws_bytes), _stream()), "sa_conv1_bwd")
+            if lv.c_in:
+                pts = cur_pts.reshape(B * lv.n, lv.c_in)
+                gU = _plain_grad(lv.dU)
+                wf = L0.W[3:]
+                self._c(lib.psa_train_dense_bwd_weight(B * lv.n, lv.c_in, L0.N, C.byref(_raw_in(pts)), C.byref(gU), _p(L0.dW[3:]), _p(self.ws),
+                                                       C.c_size_t(self.ws_bytes), _stream()), "train_dense_bwd_weight")
+                self._c(lib.psa_train_dense_bwd_input(B * lv.n, lv.c_in, L0.N, C.byref(gU), _p(wf), _p(lv.d_in), lv.c_in, 0, _p(self.ws),
+                                                      C.c_size_t(self.ws_bytes), _stream()), "train_dense_bwd_input")
+
+    def backward(self, dlogits: torch.Tensor):
+        """Gradients of every trainable variable for d(loss)/d(logits) = dlogits, into the flat gradient bucket."""
         # ---- head ----  (a bare level stack: dlogits is the gradient of the last level's pooled features)
         dh = dlogits.contiguous()
         if not self.head:
@@ -473,43 +525,8 @@ class PointNet2ClsTrainer(_TrainOps):
         # ---- set-abstraction levels, last to first ----
         dpool = self.d_feat
         for li in range(len(self.levels) - 1, -1, -1):
-            lv = self.levels[li]
-            sp = lv.spec
-            L = len(lv.layers)
-            cur_xyz, cur_pts = self.in_xyz[li]
-            for l in range(L - 1, 0, -1):
-                ly = lv.layers[l]
-                if l == L - 1:
-                    g0 = _grad_pooled(ly, dpool, lv.pooled, lv.argk, lv.k, False)
-                    g1 = _grad_pooled(ly, dpool, lv.pooled, lv.argk, lv.k, True)
-                else:
-                    g0 = _grad_dense(ly, lv.dh[l], False)
-                    g1 = _grad_dense(ly, lv.dh[l], True)
-                self._layer_bwd(ly, g0, g1, lv.layers[l - 1].act_in(), lv.dh[l - 1])
-            L0 = lv.layers[0]
-            if L == 1:
-                g0 = _grad_pooled(L0, dpool, lv.pooled, lv.argk, lv.k, False)
-                g1 = _grad_pooled(L0, dpool, lv.pooled, lv.argk, lv.k, True)
-            else:
-                g0 = _grad_dense(L0, lv.dh[0], False)
-                g1 = _grad_dense(L0, lv.dh[0], True)
-            if sp.group_all:
-                self._layer_bwd(L0, g0, g1, _raw_in(lv.x_cat), lv.d_in, col_skip=3)
-            else:
-                self._c(lib.psa_bn_bwd_coeffs(L0.rows, L0.N, C.byref(g0), _p(L0.gamma), _p(L0.mean_inv), _p(L0.dgamma), _p(L0.dbeta),
-                                              _p(L0.ca), _p(L0.cb), _p(L0.cc), _p(self.ws), C.c_size_t(self.ws_bytes), _stream()), "bn_bwd_coeffs")
-                L0.db.zero_()
-                self._c(lib.psa_sa_conv1_bwd(B, lv.n, lv.m, lv.k, L0.N, _p(cur_xyz), _p(lv.new_xyz), _p(lv.idx), C.byref(g1), _p(L0.dW[:3]),
-                                             _p(lv.dU), _p(self.ws), C.c_size_t(self.ws_bytes), _stream()), "sa_conv1_bwd")
-                if lv.c_in:
-                    pts = cur_pts.reshape(B * lv.n, lv.c_in)
-                    gU = _plain_grad(lv.dU)
-                    wf = L0.W[3:]
-                    self._c(lib.psa_train_dense_bwd_weight(B * lv.n, lv.c_in, L0.N, C.byref(_raw_in(pts)), C.byref(gU), _p(L0.dW[3:]), _p(self.ws),
-                                                           C.c_size_t(self.ws_bytes), _stream()), "train_dense_bwd_weight")
-                    self._c(lib.psa_train_dense_bwd_input(B * lv.n, lv.c_in, L0.N, C.byref(gU), _p(wf), _p(lv.d_in), lv.c_in, 0, _p(self.ws),
-                                                          C.c_size_t(self.ws_bytes), _stream()), "train_dense_bwd_input")
-            dpool = lv.d_in
+            self._level_backward(li, dpool)
+            dpool = self.levels[li].d_in
 
     # ------------------------------------------------------------------------------------------------
     def loss_and_grad(self, logits: torch.Tensor, labels: torch.Tensor):
@@ -536,6 +553,252 @@ class PointNet2ClsTrainer(_TrainOps):
         logits = self.forward(xyz, bn_decay)
         loss, dl = self.loss_and_grad(logits, labels)
         self.backward(dl)
+        self.allreduce_grads()
+        self.adam(lr)
+        return loss
+
+
+@dataclass
+class FpSpec:
+    """One pointnet_fp_module call (pointnet2_cls_bga.py:51-53)."""
+    scope: str
+    mlp: list
+
+
+# pointnet2_cls_bga.py:30-67 (SA1 takes nsample 64 here, 32 in pointnet2_cls_ssg)
+BGA_LEVELS = [LevelSpec("layer1", 512, 0.2, 64, [64, 64, 128]), LevelSpec("layer2", 128, 0.4, 64, [128, 128, 256]),
+              LevelSpec("layer3", None, None, None, [256, 512, 1024], group_all=True)]
+BGA_FP = [FpSpec("fa_layer1", [256, 256]), FpSpec("fa_layer2", [256, 128]), FpSpec("fa_layer3", [128, 128, 128])]
+BGA_SEG_HEAD = [("seg_fc1", 128, True, 0.5), ("seg_fc2", 2, False, None)]      # (scope, width, bn, keep_prob)
+
+
+@dataclass
+class _Fp:
+    """buffers of one feature-propagation module: n unknown / m known points per cloud, c_a interpolated and c_s skip channels"""
+    spec: FpSpec
+    n: int
+    m: int
+    c_a: int
+    c_s: int
+    layers: list = field(default_factory=list)
+    U: torch.Tensor = None                      # (B*m, C1) = P2 . W1[:c_a]
+    idx: torch.Tensor = None                    # (B, n, 3)
+    weight: torch.Tensor = None                 # (B, n, 3)
+    dh: list = field(default_factory=list)      # dh[l] = gradient w.r.t. layer l's post-relu output, l < L-1
+    dU: torch.Tensor = None                     # (B*m, C1)
+    dP2: torch.Tensor = None                    # (B*m, c_a): gradient w.r.t. the interpolated features' source
+    dskip: torch.Tensor = None                  # (B*n, c_s)
+    p2_in: PsaActIn = None                      # the forward's P2 operand (kept for the weight gradient)
+    skip: torch.Tensor = None
+
+
+class PointNet2BgaTrainer(PointNet2ClsTrainer):
+    """Training engine of pointnet2_cls_bga (classification + background-mask segmentation): one sess.run(train_op) of
+    pointnet2/train_seg.py on the hand-written kernels.  The set-abstraction levels and the FC head are PointNet2ClsTrainer's; the
+    feature-propagation modules never build the interpolated or concatenated inputs (psa_fp_conv1_prebn / psa_fp_conv1_bwd), the
+    joint loss is psa_cls_seg_xent.  Three tensors feed two consumers each, and their gradients are summed before their producer's
+    backward: l2_points (SA3 and fa_layer1's skip), l1_points (SA2 and fa_layer2's skip), fc2's activated output (fc3 through the dp2
+    mask, fa_layer1 without it: class_vector is tapped before dp2, pointnet2_cls_bga.py:45-48)."""
+
+    def __init__(self, params: VariableStore, batch: int, npoints: int, num_class: int = 15, device=None, process_group=None,
+                 levels=None):
+        super().__init__(params, batch, npoints, num_class, levels=levels if levels is not None else BGA_LEVELS, head=SSG_HEAD,
+                         device=device, process_group=process_group)
+        assert len(self.levels) == 3 and self.levels[2].spec.group_all and len(self.head) == 3
+        lib = self.lib
+        dev = self.dev
+        f32 = dict(dtype=torch.float32, device=dev)
+        B = batch
+        lv1, lv2, _ = self.levels
+        fc2 = self.head[1]
+        ws_bytes = self.ws_bytes
+        # pointnet2_cls_bga.py:51-53: (unknown points, known points, skip channels); interpolated channels = the producer's width
+        wiring = [(lv2.m, 1, lv2.spec.mlp[-1]), (lv1.m, lv2.m, lv1.spec.mlp[-1]), (npoints, lv1.m, 0)]
+        self.fps: list[_Fp] = []
+        c_a = fc2.N
+        for sp, (n, m, c_s) in zip(BGA_FP, wiring):
+            f = _Fp(sp, n, m, c_a, c_s)
+            cin = c_a + c_s
+            for i, cout in enumerate(sp.mlp):
+                ly = _Layer(self.fp, f"{sp.scope}/conv_{i}", B * n, True, dev)
+                assert ly.K == cin and ly.N == cout, (sp.scope, i, ly.W.shape, cin, cout)
+                ws_bytes = max(ws_bytes, lib.psa_train_dense_workspace_bytes(B * n, cin, cout), lib.psa_bn_bwd_workspace_bytes(cout))
+                f.layers.append(ly)
+                cin = cout
+            c1 = sp.mlp[0]
+            ws_bytes = max(ws_bytes, lib.psa_train_dense_workspace_bytes(B * m, c_a, c1), lib.psa_fp_conv1_prebn_workspace_bytes(B, n, c1),
+                           lib.psa_fp_conv1_bwd_workspace_bytes(B, n, m))
+            if c_s:
+                ws_bytes = max(ws_bytes, lib.psa_train_dense_workspace_bytes(B * n, c_s, c1))
+                f.dskip = torch.empty((B * n, c_s), **f32)
+            f.U = torch.empty((B * m, c1), **f32)
+            f.dU = torch.empty((B * m, c1), **f32)
+            f.dP2 = torch.empty((B * m, c_a), **f32)
+            f.idx = torch.empty((B, n, 3), dtype=torch.int32, device=dev)
+            f.weight = torch.empty((B, n, 3), **f32)
+            f.dh = [torch.empty((B * n, w), **f32) for w in sp.mlp[:-1]]
+            self.fps.append(f)
+            c_a = sp.mlp[-1]
+        # per-point segmentation head on the B*N rows of fa_layer3's output
+        self.seg: list[_Layer] = []
+        self.seg_keep: list = []
+        rows = B * npoints
+        cin = c_a
+        for scope, width, bn, keep in BGA_SEG_HEAD:
+            ly = _Layer(self.fp, scope, rows, bn, dev)
+            assert ly.K == cin and ly.N == width, (scope, ly.W.shape)
+            if keep is not None:
+                ly.mask = torch.ones((rows, width), **f32)
+            ws_bytes = max(ws_bytes, lib.psa_train_dense_workspace_bytes(rows, cin, width), lib.psa_bn_bwd_workspace_bytes(width))
+            self.seg.append(ly)
+            self.seg_keep.append(keep)
+            cin = width
+        self.seg_dh = torch.empty((rows, self.seg[0].N), **f32)        # gradient w.r.t. seg_fc1's (masked) output
+        self.fp_dout = torch.empty((rows, c_a), **f32)                 # gradient w.r.t. fa_layer3's output
+        self.d_h2 = torch.empty((B, fc2.N), **f32)                      # gradient w.r.t. fc2's activated output (both consumers)
+        self.dseg = torch.empty((rows, 2), **f32)
+        self.loss = torch.zeros(3, **f32)
+        ws_bytes = max(ws_bytes, lib.psa_cls_seg_xent_workspace_bytes(B, npoints))
+        if ws_bytes > self.ws_bytes:
+            self.ws = torch.empty(ws_bytes // 4 + 64, **f32)
+            self.ws_bytes = ws_bytes
+
+    # ------------------------------------------------------------------------------------------------
+    def _masked(self):
+        return [(ly, keep) for ly, keep in zip(self.head + self.seg, self.keep + self.seg_keep) if keep is not None]
+
+    def draw_dropout(self):
+        """tf.nn.dropout masks of dp1, dp2 and seg_dp1 (0 or 1/keep_prob), drawn on the device before the step."""
+        for ly, keep in self._masked():
+            r = torch.rand(ly.mask.shape, generator=self._gen, device=self.dev)
+            ly.mask.copy_((r < keep).to(torch.float32) / keep)
+
+    def _fp_forward(self, f: _Fp, xyz1: torch.Tensor, xyz2: torch.Tensor, p2_in: PsaActIn, skip: torch.Tensor | None, bn_decay: float):
+        lib = self.lib
+        B = self.B
+        L0 = f.layers[0]
+        f.p2_in, f.skip = p2_in, skip
+        self._c(lib.psa_train_dense_fwd(B * f.m, f.c_a, L0.N, C.byref(p2_in), _p(L0.W[:f.c_a]), None, _p(f.U), None, _p(self.ws),
+                                        C.c_size_t(self.ws_bytes), _stream()), "train_dense_fwd")
+        if skip is not None:
+            self._c(lib.psa_train_dense_fwd(B * f.n, f.c_s, L0.N, C.byref(_raw_in(skip)), _p(L0.W[f.c_a:]), _p(L0.b), _p(L0.y), None,
+                                            _p(self.ws), C.c_size_t(self.ws_bytes), _stream()), "train_dense_fwd")
+        self._c(lib.psa_fp_conv1_prebn(B, f.n, f.m, L0.N, _p(xyz1), _p(xyz2), _p(f.U), _p(L0.b), 1 if skip is not None else 0, _p(L0.y),
+                                       _p(f.idx), _p(f.weight), _p(L0.stats), _p(self.ws), C.c_size_t(self.ws_bytes), _stream()),
+                "fp_conv1_prebn")
+        self._bn_finalize(L0, L0.rows, bn_decay)
+        prev = L0
+        for ly in f.layers[1:]:
+            self._dense_fwd(ly, prev.act_in())
+            self._bn_finalize(ly, ly.rows, bn_decay)
+            prev = ly
+
+    def _fps_forward(self, bn_decay: float):
+        """fa_layer1..3 (pointnet2_cls_bga.py:51-53) after the levels and the FC head have run"""
+        lv1, lv2, lv3 = self.levels
+        p2 = self.head[1].act_in()
+        p2.mask = None                                   # class_vector: fc2's output before dp2
+        self._fp_forward(self.fps[0], lv2.new_xyz, lv3.new_xyz, p2, lv2.pooled, bn_decay)
+        self._fp_forward(self.fps[1], lv1.new_xyz, lv2.new_xyz, self.fps[0].layers[-1].act_in(), lv1.pooled, bn_decay)
+        self._fp_forward(self.fps[2], self.in_xyz[0][0], lv1.new_xyz, self.fps[1].layers[-1].act_in(), None, bn_decay)
+
+    def _seg_forward(self, bn_decay: float):
+        """seg_fc1 -> seg_dp1 -> seg_fc2 on fa_layer3's output"""
+        a = self.fps[2].layers[-1].act_in()
+        for ly in self.seg:
+            self._dense_fwd(ly, a)
+            if ly.bn:
+                self._bn_finalize(ly, ly.rows, bn_decay)
+            a = ly.act_in()
+
+    def forward(self, xyz: torch.Tensor, bn_decay: float = 0.5):
+        """Training-mode forward (batch statistics, moving averages updated with `bn_decay`) -> (class logits (B, num_class),
+        seg logits (B, N, 2))."""
+        B = self.B
+        class_logits = super().forward(xyz, bn_decay)
+        self._fps_forward(bn_decay)
+        self._seg_forward(bn_decay)
+        return class_logits, self.seg[-1].y.view(B, self.N0, -1)
+
+    # ------------------------------------------------------------------------------------------------
+    def loss_and_grad(self, class_logits: torch.Tensor, seg_logits: torch.Tensor, labels: torch.Tensor, mask: torch.Tensor,
+                      seg_weight: float = 0.5):
+        """pointnet2_cls_bga.get_loss (pointnet2_cls_bga.py:78-93) -> loss (3,) = [total, classify, seg], d loss / d class_logits,
+        d loss / d seg_logits.  labels (B,) and mask (B, N) int32."""
+        assert labels.dtype == torch.int32 and mask.dtype == torch.int32 and mask.shape == (self.B, self.N0)
+        self._c(self.lib.psa_cls_seg_xent(self.B, self.num_class, self.N0, _p(class_logits), _p(labels), _p(seg_logits), _p(mask),
+                                          C.c_float(seg_weight), _p(self.loss), _p(self.dlogits), _p(self.dseg), _p(self.ws),
+                                          C.c_size_t(self.ws_bytes), _stream()), "cls_seg_xent")
+        return self.loss, self.dlogits, self.dseg.view(self.B, self.N0, 2)
+
+    def _fp_backward(self, f: _Fp, dout: torch.Tensor):
+        """gradients of one FP module's variables for d(loss)/d(output) = dout -> f.dP2 (and f.dskip)"""
+        lib = self.lib
+        B = self.B
+        L = len(f.layers)
+        for l in range(L - 1, 0, -1):
+            ly = f.layers[l]
+            dh = dout if l == L - 1 else f.dh[l]
+            self._layer_bwd(ly, _grad_dense(ly, dh, False), _grad_dense(ly, dh, True), f.layers[l - 1].act_in(), f.dh[l - 1])
+        L0 = f.layers[0]
+        dh = dout if L == 1 else f.dh[0]
+        g1 = _grad_dense(L0, dh, True)
+        self._layer_bwd(L0, _grad_dense(L0, dh, False), g1, None, None)          # batch-norm sums and coefficients
+        self._c(lib.psa_fp_conv1_bwd(B, f.n, f.m, L0.N, _p(f.idx), _p(f.weight), C.byref(g1), _p(f.dU), _p(self.ws),
+                                     C.c_size_t(self.ws_bytes), _stream()), "fp_conv1_bwd")
+        gU = _plain_grad(f.dU)
+        self._c(lib.psa_train_dense_bwd_weight(B * f.m, f.c_a, L0.N, C.byref(f.p2_in), C.byref(gU), _p(L0.dW[:f.c_a]), _p(self.ws),
+                                               C.c_size_t(self.ws_bytes), _stream()), "train_dense_bwd_weight")
+        self._c(lib.psa_train_dense_bwd_input(B * f.m, f.c_a, L0.N, C.byref(gU), _p(L0.W[:f.c_a]), _p(f.dP2), f.c_a, 0, _p(self.ws),
+                                              C.c_size_t(self.ws_bytes), _stream()), "train_dense_bwd_input")
+        if f.c_s:
+            self._c(lib.psa_train_dense_bwd_weight(B * f.n, f.c_s, L0.N, C.byref(_raw_in(f.skip)), C.byref(g1), _p(L0.dW[f.c_a:]),
+                                                   _p(self.ws), C.c_size_t(self.ws_bytes), _stream()), "train_dense_bwd_weight")
+            self._c(lib.psa_train_dense_bwd_input(B * f.n, L0.K, L0.N, C.byref(g1), _p(L0.W), _p(f.dskip), f.c_s, f.c_a, _p(self.ws),
+                                                  C.c_size_t(self.ws_bytes), _stream()), "train_dense_bwd_input")
+
+    def backward(self, dcls: torch.Tensor, dseg: torch.Tensor):
+        """Gradients of every trainable variable for d(loss)/d(class logits) = dcls and d(loss)/d(seg logits) = dseg, into the flat
+        gradient bucket."""
+        dseg = dseg.reshape(-1, 2).contiguous()
+        s1, s2 = self.seg
+        fa3_out = self.fps[2].layers[-1].act_in()
+        self._layer_bwd(s2, _grad_dense(s2, dseg, False), _grad_dense(s2, dseg, True), s1.act_in(), self.seg_dh)
+        self._layer_bwd(s1, _grad_dense(s1, self.seg_dh, False), _grad_dense(s1, self.seg_dh, True), fa3_out, self.fp_dout)
+        dout = self.fp_dout
+        for f in reversed(self.fps):
+            self._fp_backward(f, dout)
+            dout = f.dP2
+        fc1, fc2, fc3 = self.head
+        self._layer_bwd(fc3, _grad_dense(fc3, dcls, False), _grad_dense(fc3, dcls, True), fc2.act_in(), self.head_dh[1])
+        # fc2's activated output h2 feeds fc3 through the dp2 mask and fa_layer1 directly: d h2 = mask * dx_fc3 + dP2
+        torch.addcmul(self.fps[0].dP2, fc2.mask, self.head_dh[1], out=self.d_h2)
+        g0, g1 = _grad_dense(fc2, self.d_h2, False), _grad_dense(fc2, self.d_h2, True)
+        g0.mask = None
+        g1.mask = None
+        self._layer_bwd(fc2, g0, g1, fc1.act_in(), self.head_dh[0])
+        self._layer_bwd(fc1, _grad_dense(fc1, self.head_dh[0], False), _grad_dense(fc1, self.head_dh[0], True),
+                        _raw_in(self.levels[-1].pooled), self.d_feat)
+        # set-abstraction levels; l2_points / l1_points also fed fa_layer1 / fa_layer2 as skip features
+        _, lv2, lv3 = self.levels
+        self._level_backward(2, self.d_feat)
+        lv3.d_in.add_(self.fps[0].dskip)
+        self._level_backward(1, lv3.d_in)
+        lv2.d_in.add_(self.fps[1].dskip)
+        self._level_backward(0, lv2.d_in)
+
+    def train_step(self, xyz: torch.Tensor, labels: torch.Tensor, mask: torch.Tensor, lr: float = 1e-3, bn_decay: float = 0.5,
+                   seg_weight: float = 0.5, dropout: bool = True):
+        """one sess.run(train_op) of pointnet2/train_seg.py: forward, joint loss, backward, (all-reduce), Adam.  dropout=False runs
+        with every keep mask at 1.  -> loss (3,) = [total, classify, seg]"""
+        if dropout:
+            self.draw_dropout()
+        else:
+            for ly, _ in self._masked():
+                ly.mask.fill_(1.0)
+        class_logits, seg_logits = self.forward(xyz, bn_decay)
+        loss, dcls, dseg = self.loss_and_grad(class_logits, seg_logits, labels, mask, seg_weight)
+        self.backward(dcls, dseg)
         self.allreduce_grads()
         self.adam(lr)
         return loss
